@@ -11,11 +11,15 @@ discriminator on the 58 masked mgc dims (58-256-256-256-1), B=32 x T=1000 padded
 dropout 0.5 in train mode, full-length utterances.  cfg3 = VC In2OutRNNHighwayNet (3 x 512 BiLSTM) + MLP D, B=16 x
 T=2000; cfg5 = TTS LSTMRNN (3 x 512 BiLSTM) + MLP D + MGE, B=64 x T=1500 per GPU.
 
-Timing: W untimed warm-up steps, then the K-step loop is timed with CUDA events between barriers; the loop is
-REPEATED until at least 0.5 s of timed work has accumulated (>= 3 repeats) and the MEDIAN repeat is reported
-(`steps` stays K; a 20-step loop of a 1.3 ms step is 0.03 s, too short to be stable on its own).
+Timing: W untimed warm-up steps, then exactly K steps are timed with CUDA events between barriers (pick K so that
+the window lasts a second or more: a 20-step window of a 1.3 ms step is 0.03 s and measures mostly noise).
 
-One JSON line on stdout (rank 0); see the task contract for the keys.
+--dump-outputs DIR: after the timed steps, what the last of them computed -- the losses, y_hat and y_hat_static the
+step hands its caller and the generator and discriminator parameters it updated -- is written as DIR/<name>.npy
+(float32; a fixed seeded sample of the elements where the whole would exceed 64 MB).  Inputs and initial weights are
+seeded, so two builds run with the same arguments can be compared output for output.
+
+One JSON line on stdout (rank 0).
 """
 import argparse
 import ctypes
@@ -30,6 +34,7 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True       # the tree may be read-only; the benchmark writes nothing into it
 sys.path.insert(0, ROOT)
 sys.path.insert(1, os.path.join(ROOT, "compat"))
 
@@ -55,8 +60,8 @@ WORKLOADS = {
                       "mask_nth=2), B=64 T=1500 per GPU, MGE(MLPG)+ADV, Adagrad"),
 }
 NUM_BATCHES = 4          # ring of distinct synthetic batches (larger than the 126 MB L2 for every workload)
-MIN_TIMED_SECONDS = 0.5
-MAX_REPEATS = 25
+DUMP_BYTES = 64 << 20    # --dump-outputs: at most this much in all
+NPY_HEADER_BYTES = 128
 
 
 def algorithmic_flops_per_frame(w):
@@ -94,6 +99,22 @@ def make_batches(w, seed, n, pinned, B=None):
             x, y = x.pin_memory(), y.pin_memory()
         out.append((x, y))
     return out
+
+
+def dump_outputs(arrays, out_dir, budget=DUMP_BYTES):
+    """Write {name: float32/float64 array} as out_dir/<name>.npy, at most `budget` bytes in all.  Smallest first, each
+    array gets an equal share of what is left; one that does not fit is replaced by a sample of its flattened
+    elements, drawn with a fixed seed and kept in index order, so runs with the same shapes sample the same elements."""
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: (kv[1].nbytes, kv[0]))
+    left = budget
+    for i, (name, a) in enumerate(items):
+        share = left // (len(items) - i) - NPY_HEADER_BYTES
+        if a.nbytes > share:
+            idx = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes + NPY_HEADER_BYTES
 
 
 class ClockSampler(object):
@@ -303,8 +324,8 @@ def workload_config(w, engine, args=None):
     return {"workload": w["text"], "global_batch_per_gpu": w["B"], "seq_len": w["T"], "engine": engine,
             "l2": "per-step working set > 1 GB and a ring of %d distinct input batches (%d MB) exceed the 126 MB L2; "
                   "no explicit flush" % (NUM_BATCHES, NUM_BATCHES * bytes_per_batch // (1 << 20)),
-            "timing": "median of R repeats of the K-step loop (>= 3 repeats and >= %.1f s of timed work), CUDA "
-                      "events, barrier + synchronize on both sides, max over ranks" % MIN_TIMED_SECONDS,
+            "timing": "one window of exactly K = --steps steps, CUDA events, barrier + synchronize on both sides, "
+                      "max over ranks",
             "parallelism": "utterance-sharded data parallel, one NCCL SUM all-reduce per model per step"}
 
 
@@ -350,7 +371,6 @@ def run_b200_arm(args):
     if os.environ.get("GANTTS_B200_DBG", "0") not in ("", "0") or os.environ.get("GANTTS_B200_CHAIN_DBG", "0") not in ("", "0"):
         raise SystemExit("bench.py: GANTTS_B200_DBG is a phase-timing switch that skips work inside the kernels; "
                          "refusing to produce a benchmark line with it set")
-    import __graft_entry__
     from gantts_b200 import parallel
     # stdout carries exactly ONE JSON line.  NCCL prints its version banner with a bare printf on fd 1 during
     # the first communicator init (NCCL_DEBUG_FILE does not catch it), so fd 1 points at stderr for the whole
@@ -362,10 +382,8 @@ def run_b200_arm(args):
         raise SystemExit("bench.py: no CUDA device -- the B200 arm has no CPU fallback")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
-    if rank == 0:
-        __graft_entry__.build()
-    if world > 1:
-        torch.distributed.barrier()
+    # the library comes from `python -m gantts_b200.build` (or __graft_entry__.build()); the benchmark only loads
+    # it, so it runs from a read-only tree
     import gantts_b200
     from gantts_b200 import _lib, step as gstep, config
     from nnmnkwii.paramgen import unit_variance_mlpg_matrix   # compat shim (product side, memoised)
@@ -399,7 +417,21 @@ def run_b200_arm(args):
             if path == "fused":
                 losses = self.fs.step(x, y, lengths, frames=frames_per_step)
                 return {"loss_d": losses[0], "loss_mge": losses[4], "loss_adv": losses[5], "loss_g": losses[6]}
-            return self.tr.step(x, y, lengths, self.R)[0]
+            self.last = self.tr.step(x, y, lengths, self.R)
+            return self.last[0]
+
+        def outputs(self):
+            """What the last step handed its caller, and the parameters it updated: {name: float32 array}."""
+            if path == "fused":
+                from gantts_b200.fused import LOSS_NAMES
+                out = dict(zip(LOSS_NAMES, self.fs.losses.detach().cpu().unbind()))
+                out["y_hat"], out["y_hat_static"] = self.fs.y_hat, self.fs.y_hat_static
+            else:
+                out = dict(self.last[0])
+                out["y_hat"], out["y_hat_static"] = self.last[1], self.last[2]
+            for tag, m in (("g", mg), ("d", md)):
+                out.update(("%s.%s" % (tag, k), p) for k, p in m.named_parameters())
+            return {k: torch.as_tensor(v).detach().float().cpu().numpy() for k, v in out.items()}
 
         def nccl_warmup(self):
             if world == 1:
@@ -429,34 +461,22 @@ def run_b200_arm(args):
 
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 
-    def timed_repeats(loop):
-        """loop(K) enqueues K steps; returns (median ms per step, list of per-repeat ms per step)."""
-        per, total = [], 0.0
-        while True:
-            barrier()
-            t_host = time.perf_counter()
-            e0.record()
-            loop(args.steps)
-            e1.record()
-            t_host = time.perf_counter() - t_host
-            barrier()
-            local_ms = e0.elapsed_time(e1)
-            ms = max_over_ranks(local_ms)
-            if os.environ.get("GANTTS_B200_BENCH_TRACE"):
-                sys.stderr.write("[trace] rank %d repeat %d: device %.3f ms/step (max over ranks %.3f), host enqueue %.3f ms/step\n"
-                                 % (rank, len(per), local_ms / args.steps, ms / args.steps, t_host / args.steps * 1e3))
-                sys.stderr.flush()
-            per.append(ms / args.steps)
-            total += ms
-            enough = len(per) >= 3 and total >= MIN_TIMED_SECONDS * 1e3
-            # a transient on the box (one 2-GPU run of round 2 saw repeats of 1.2, 8 and 16 ms/step, none of the following
-            # runs did): while the repeats disagree by more than 30 %, keep measuring (bounded) so the median is not
-            # decided by three samples
-            if enough and max(per) > 1.3 * min(per) and len(per) < 11 and total < 8e3:
-                enough = False
-            if enough or len(per) >= MAX_REPEATS:
-                break
-        return float(np.median(per)), per
+    def timed(loop):
+        """loop(K) enqueues K = --steps steps; returns ms per step over that one window (max over ranks)."""
+        barrier()
+        t_host = time.perf_counter()
+        e0.record()
+        loop(args.steps)
+        e1.record()
+        t_host = time.perf_counter() - t_host
+        barrier()
+        local_ms = e0.elapsed_time(e1)
+        ms = max_over_ranks(local_ms)
+        if os.environ.get("GANTTS_B200_BENCH_TRACE"):
+            sys.stderr.write("[trace] rank %d: device %.3f ms/step (max over ranks %.3f), host enqueue %.3f ms/step\n"
+                             % (rank, local_ms / args.steps, ms / args.steps, t_host / args.steps * 1e3))
+            sys.stderr.flush()
+        return ms / args.steps
 
     # ---------------- value: inputs resident in HBM
     trainer.nccl_warmup()
@@ -481,9 +501,11 @@ def run_b200_arm(args):
             last["out"] = trainer.step(*resident[i % NUM_BATCHES])
 
     launches0 = lib.gantts_launch_count()
-    ms_per_step, repeats = timed_repeats(resident_loop)
-    launches = (lib.gantts_launch_count() - launches0) / float(len(repeats) * args.steps)
+    ms_per_step = timed(resident_loop)
+    launches = (lib.gantts_launch_count() - launches0) / float(args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(trainer.outputs(), args.dump_outputs)
     value = frames_per_step / (ms_per_step * 1e-3)
     loss_g = float(last["out"]["loss_g"])
     # host time to ENQUEUE a step (8 steps stay well inside the driver's launch queue, so the CPU never waits for the
@@ -533,7 +555,7 @@ def run_b200_arm(args):
     for ev in consumed:
         ev.record()
     e2e_loop(max(2, min(args.warmup, 4)))
-    e2e_ms, e2e_repeats = timed_repeats(e2e_loop)
+    e2e_ms = timed(e2e_loop)
     h2d = sum(t.numel() * 4 for t in host[0])
 
     # ---------------- N > 1: what the two gradient all-reduces of a step cost by themselves (back to back, no skew to
@@ -549,7 +571,7 @@ def run_b200_arm(args):
                     b.mul_(1.0 / world)             # keeps the values bounded over the repeats
 
         ar_loop(5)
-        ar_ms, _ = timed_repeats(ar_loop)
+        ar_ms = timed(ar_loop)
         allreduce = {"us_per_step_pair": ar_ms * 1e3, "d_bytes": gbufs[0].numel() * 4, "g_bytes": gbufs[1].numel() * 4,
                      "note": "D + G gradient all-reduce (NCCL) + one scale kernel each, timed alone"}
 
@@ -644,10 +666,8 @@ def run_b200_arm(args):
             "scaling": "weak", "vs_baseline": None,
             "dtype": "f32 (GEMMs: bf16x3 split on tcgen05, fp32 accumulate)" if args.engine == "tc" else "f32",
             "data": "synthetic", "config": workload_config(w, args.engine, args), "clocks": clocks,
-            "timed_repeats": {"n": len(repeats), "ms_per_step_min": min(repeats), "ms_per_step_max": max(repeats),
-                              "ms_per_step_all": [round(v, 4) for v in repeats]},
             "e2e": {"value": frames_per_step / (e2e_ms * 1e-3), "unit": "frames/s", "ms_per_step": e2e_ms,
-                    "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 16, "repeats": len(e2e_repeats),
+                    "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 16,
                     "how": "pinned host x,y -> double-buffered cudaMemcpyAsync on a copy stream -> one step through the "
                            "public API (%s) -> 4 loss scalars D2H; copies inside the timed region" % path},
             "gpu_launches": int(round(launches * args.steps)), "gpu_launches_per_step": launches,
@@ -676,10 +696,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-dropin", action="store_true")
     ap.add_argument("--path", default="fused", choices=["fused", "modular"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
-    if args.workload != "cfg2" and args.steps > 10:
-        args.steps = 10                    # recurrent workloads: ~0.1 - 1 s per step
     if args.impl == "reference":
         run_reference_arm(args)
     else:

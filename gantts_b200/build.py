@@ -12,9 +12,10 @@ FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std
 
 
 def sources():
+    """The files the library is compiled from (not the .ptxas.log that build() writes next to them after linking)."""
     d = os.path.join(HERE, "csrc")
     inc = os.path.join(os.path.dirname(HERE), "include")
-    return [os.path.join(d, f) for f in os.listdir(d)] + [os.path.join(inc, f) for f in os.listdir(inc)]
+    return [os.path.join(p, f) for p in (d, inc) for f in os.listdir(p) if f.endswith((".cu", ".cuh", ".h"))]
 
 
 def up_to_date():

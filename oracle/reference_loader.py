@@ -1,8 +1,8 @@
 """Import the UNMODIFIED reference Python (r9y9/gantts) from /root/reference.  TEST INFRASTRUCTURE.
 
-Only usable in the build container (``/root/reference`` does not exist on the GPU box); it is
-what ``tests/golden/make_golden.py`` uses to generate the committed golden vectors and what the
-``not gpu`` tests use (when the tree is present) to re-pin ``oracle.gantts_port``.
+Only usable where the reference tree is present (``GANTTS_REFERENCE_ROOT``); it is what
+``tests/golden/make_golden.py`` uses to generate the committed golden vectors.  The tests read
+only those vectors, so they run without the reference.
 
 The reference does not import as shipped (SURVEY.md section 8c): ``gantts/__init__.py:4`` needs
 a generated ``gantts/version.py`` (setup.py:24-36), ``multistream.py:11-12``/``models.py:8``

@@ -12,6 +12,7 @@ oracle/nnmnkwii_port.py (nnmnkwii itself is not installable offline: "parity unp
 third-party arithmetic, see oracle/__init__.py).  Inputs and weights are stored next to the
 outputs so the tests do not depend on torch's RNG stream staying stable across versions.
 """
+import json
 import os
 import sys
 
@@ -304,10 +305,98 @@ def gen_eval(ref, out):
             out["eval_%s_%s" % (tag, k)] = np.asarray(v, dtype=np.float64)
 
 
+def run_reference_unit_tests(ref):
+    """Execute the reference's own tests/test_gantts.py (5 tests) where it lies, on top of the nnmnkwii restatement."""
+    import importlib.util
+    import types
+    stubs = reference_loader._stub_modules()
+    names = list(stubs) + ["gantts", "gantts.models", "gantts.seqloss", "gantts.multistream"]
+    saved = {k: sys.modules.get(k) for k in names}
+    try:
+        sys.modules.update(stubs)
+        pkg = types.ModuleType("gantts")
+        pkg.models, pkg.seqloss, pkg.multistream = ref.models, ref.seqloss, ref.multistream
+        sys.modules.update({"gantts": pkg, "gantts.models": ref.models,
+                            "gantts.seqloss": ref.seqloss, "gantts.multistream": ref.multistream})
+        path = os.path.join(reference_loader.REFERENCE_ROOT, "tests", "test_gantts.py")
+        spec = importlib.util.spec_from_file_location("_ref_test_gantts", path)
+        mod = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(mod)
+        ran = 0
+        for name in sorted(dir(mod)):
+            if name.startswith("test_"):
+                getattr(mod, name)()
+                ran += 1
+        assert ran == 5
+    finally:
+        for k, v in saved.items():
+            if v is None:
+                sys.modules.pop(k, None)
+            else:
+                sys.modules[k] = v
+
+
+def gen_selftests(ref, out):
+    """What the reference computes on the inputs of tests/test_reference_selftests.py (the configurations of the
+    reference's tests/test_gantts.py), after checking that those 5 reference tests pass."""
+    sys.path.insert(0, os.path.dirname(HERE))
+    import test_reference_selftests as st
+    run_reference_unit_tests(ref)
+    ms = ref.multistream
+    sd, x1, xb, yb, lengths = st.model_case()
+    model = ref.models.In2OutHighwayNet()
+    model.load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()})
+    model.eval()
+    R = torch.from_numpy(nnp.unit_variance_mlpg_matrix(WINDOWS[:2], 100))
+    out["model_y_static"] = npy(model(torch.from_numpy(x1), R)[1])
+    x = torch.from_numpy(xb).requires_grad_(True)
+    _, y_hat = model(x, R)
+    loss = ref.seqloss.MaskedMSELoss()(y_hat, torch.from_numpy(yb), torch.from_numpy(lengths))
+    loss.backward()
+    out["model_loss"], out["model_grad_x"] = npy(loss), npy(x.grad)
+    a = torch.arange(0, 63).expand(2, 3, 63)
+    for code in st.SELECT_CASES:
+        out["select_" + code] = npy(ms.select_streams(a, [60, 1, 1, 1], st.streams(code)))
+    out["static_stream_sizes"] = ms.get_static_stream_sizes(st.STREAM_SIZES, st.HAS_DYNAMIC, 3)
+    s = torch.from_numpy(st.static_input())
+    for code in st.STATIC_CASES:
+        out["static_" + code] = npy(ms.get_static_features(s, 3, st.STREAM_SIZES, st.HAS_DYNAMIC,
+                                                           streams=st.streams(code)))
+    R = torch.from_numpy(nnp.unit_variance_mlpg_matrix(WINDOWS, 100))
+    out["mlpg_y"] = npy(ms.multi_stream_mlpg(torch.from_numpy(st.multistream_input()), R, st.STREAM_SIZES,
+                                             st.HAS_DYNAMIC))
+
+
+def gen_trainpy_imports():
+    """The module-level imports of the reference's train.py and hparams.py, and the model class names hparams.py
+    configures (what train.py:773-781 looks up in gantts.models): names only, read with ast."""
+    import ast
+    imports = []
+    for fname in ("train.py", "hparams.py"):
+        path = os.path.join(reference_loader.REFERENCE_ROOT, fname)
+        for node in ast.parse(open(path).read(), path).body:
+            if isinstance(node, ast.Import):
+                imports += [{"file": fname, "module": a.name, "names": []} for a in node.names]
+            elif isinstance(node, ast.ImportFrom):
+                imports.append({"file": fname, "module": node.module, "names": [a.name for a in node.names]})
+    ref = reference_loader.load()
+    models = {cfg: {k: getattr(ref.hparams, cfg).values()[k] for k in ("generator", "discriminator")}
+              for cfg in ("vc", "tts_duration", "tts_acoustic")}
+    return {"imports": imports, "models": models}
+
+
 def main():
     ref = reference_loader.load()
     torch.manual_seed(1234)
     torch.set_num_threads(1)
+    if "--only-reference-tests" in sys.argv:
+        f = {}
+        gen_selftests(ref, f)
+        np.savez_compressed(os.path.join(HERE, "selftests.npz"), **f)
+        with open(os.path.join(HERE, "trainpy_imports.json"), "w") as fh:
+            json.dump(gen_trainpy_imports(), fh, indent=1)
+        print("selftests", os.path.getsize(os.path.join(HERE, "selftests.npz")))
+        return
     if "--only-eval" in sys.argv:
         e = {}
         gen_eval(ref, e)
@@ -335,7 +424,12 @@ def main():
     e = {}
     gen_eval(ref, e)
     np.savez_compressed(os.path.join(HERE, "eval.npz"), **e)
-    for n in ("ops", "models", "step", "step_models", "eval"):
+    f = {}
+    gen_selftests(ref, f)
+    np.savez_compressed(os.path.join(HERE, "selftests.npz"), **f)
+    with open(os.path.join(HERE, "trainpy_imports.json"), "w") as fh:
+        json.dump(gen_trainpy_imports(), fh, indent=1)
+    for n in ("ops", "models", "step", "step_models", "eval", "selftests"):
         print(n, os.path.getsize(os.path.join(HERE, n + ".npz")))
 
 

@@ -1,4 +1,5 @@
 """CPU tests of the import shims that let the reference's train.py / hparams.py run unchanged on this image."""
+import json
 import os
 import subprocess
 import sys
@@ -8,7 +9,6 @@ import pytest
 
 from conftest import ROOT, WINDOWS
 from oracle import nnmnkwii_port as nnp
-from oracle import reference_loader
 
 COMPAT = os.path.join(ROOT, "compat")
 
@@ -84,16 +84,51 @@ options:
     assert docopt(doc, ["--flag", "a", "b"])["--w_d"] == "1.0"
 
 
-@pytest.mark.skipif(not reference_loader.available(), reason="reference tree not present")
+_RESOLVE_IMPORTS = r"""
+import importlib, json, sys
+sys.path[:0] = [ROOT, COMPAT]
+g = json.load(open(GOLDEN))
+where = {}
+for imp in g["imports"]:
+    if imp["module"] == "hparams":        # the reference's own configuration file, next to its train.py
+        continue
+    mod = importlib.import_module(imp["module"])
+    for name in imp["names"]:
+        obj = getattr(mod, name, None)
+        if obj is None:
+            obj = importlib.import_module(imp["module"] + "." + name)
+        where[imp["module"] + ":" + name] = getattr(obj, "__module__", None) or obj.__name__
+    where[imp["module"]] = getattr(mod, "__file__", None) or ""
+import gantts, tensorflow
+models = {"%s.%s" % (cfg, role): getattr(gantts.models, name).__module__
+          for cfg, roles in g["models"].items() for role, name in roles.items()}
+print(json.dumps({"gantts": gantts.__name__, "where": where, "models": models,
+                  "hparams_class": tensorflow.contrib.training.HParams.__module__}))
+"""
+
+
 def test_reference_train_py_imports_unchanged_on_the_alias_package():
-    """`import train` (the reference's own train.py, read in place) with PYTHONPATH = repo : repo/compat:
-    every import it makes resolves to the B200 package / shims and its model lookup finds our classes."""
-    code = ("import sys; sys.path[:0]=[%r,%r,%r]; import numpy as np; np.int=int; import train, gantts, hparams; "
-            "m=getattr(gantts.models, hparams.tts_acoustic.generator); "
-            "print(gantts.__name__, m.__module__, train.MaskedMSELoss.__module__, "
-            "train.unit_variance_mlpg_matrix.__module__, hparams.vc.generator)"
-            % (ROOT, COMPAT, reference_loader.REFERENCE_ROOT))
+    """Every module-level import of the reference's train.py and hparams.py (recorded from the unmodified files in
+    tests/golden/trainpy_imports.json) resolves with PYTHONPATH = repo : repo/compat, in a fresh interpreter: the
+    gantts.* names to the B200 package, nnmnkwii / tensorflow / docopt / tensorboard_logger to the shims, and the
+    generator / discriminator classes hparams.py names are found in gantts.models."""
+    golden = os.path.join(ROOT, "tests", "golden", "trainpy_imports.json")
+    code = "ROOT, COMPAT, GOLDEN = %r, %r, %r\n" % (ROOT, COMPAT, golden) + _RESOLVE_IMPORTS
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr[-2000:]
-    assert out.stdout.split() == ["gantts", "gantts_b200.models", "gantts_b200.seqloss", "nnmnkwii.paramgen",
-                                  "In2OutHighwayNet"]
+    got = json.loads(out.stdout.strip().splitlines()[-1])
+    assert got["gantts"] == "gantts"
+    recorded = json.load(open(golden))
+    assert {"vc", "tts_duration", "tts_acoustic"} <= set(recorded["models"])
+    assert recorded["models"]["vc"]["generator"] == "In2OutHighwayNet"
+    assert set(got["models"].values()) == {"gantts_b200.models"}, got["models"]
+    assert got["hparams_class"].startswith("tensorflow.")
+    w = got["where"]
+    assert w["gantts.seqloss:MaskedMSELoss"] == "gantts_b200.seqloss"
+    assert w["nnmnkwii.paramgen:unit_variance_mlpg_matrix"] == "nnmnkwii.paramgen"
+    for key, module in w.items():
+        name = key.split(":")[0]
+        if ":" in key and name.startswith("gantts"):
+            assert module.startswith("gantts_b200."), (key, module)
+        if ":" not in key and name.split(".")[0] in ("nnmnkwii", "tensorflow", "docopt", "tensorboard_logger"):
+            assert os.path.realpath(module).startswith(os.path.realpath(COMPAT) + os.sep), (key, module)

@@ -278,3 +278,25 @@ def test_bench_algorithmic_work_matches_survey_8d():
         F_D = sum(a * b for a, b in zip(dd[:-1], dd[1:]))
         want = 3 * (F_L + out_macs) - 2 * 4 * H * w["d_in"] + 2 * w.get("static_dim", 0) ** 2 + 8 * F_D - dd[1] * dd[0]
         assert bench.algorithmic_flops_per_frame(w) == 2.0 * want
+
+
+def test_bench_dump_outputs_budget_and_sample(tmp_path):
+    """bench.py --dump-outputs: small arrays are written whole, large ones as a seeded sample of their elements, the
+    directory stays within the budget, and the same shapes always sample the same elements."""
+    import bench
+    rs = np.random.RandomState(0)
+    arrays = {"loss_g": np.float32(rs.rand(1)), "y_hat": rs.rand(600, 187).astype(np.float32),
+              "g.w": rs.rand(512, 425).astype(np.float32), "d.b": rs.rand(256).astype(np.float64)}
+    budget = 1 << 19
+    for run in ("a", "b"):
+        bench.dump_outputs(arrays, str(tmp_path / run), budget=budget)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["d.b.npy", "g.w.npy", "loss_g.npy", "y_hat.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= budget
+    for name, a in arrays.items():
+        got, again = np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy"))
+        assert got.dtype == a.dtype and np.array_equal(got, again)
+        if name in ("loss_g", "d.b"):
+            assert np.array_equal(got, a)
+        else:
+            assert got.ndim == 1 and 0 < got.size < a.size and np.isin(got, a.reshape(-1)).all()
